@@ -68,6 +68,8 @@ SMALL_W, SMALL_H = 480, 270     # the CPU arms' bounded sample: one real small v
 SMALL_POOL = 8
 REGULARIZATION = 0.01           # app/smvsrecon.cc:712 with alpha = 1
 METRIC = "Gauss-Newton Mpix-iters/sec"
+DUMP_STATS = ("newton_steps", "cg_iterations", "pixel_iterations", "n_active")
+DUMP_LIMIT = 64 << 20           # bytes of --dump-outputs
 UNIT = "Mpix-iters/s"
 CONFIG = {
     "workload": "1 ref view + 6 neighbours, 1920x1080, scale 2 (-o2), no shading: "
@@ -462,6 +464,12 @@ def run_product(args):
     wall_resident = t1 - t0
     launches = sum(c.launches for c in ctxs) - launches0
     clocks = sampler.stop(t0, t1)
+    dump = {}
+    if args.dump_outputs and args.steps > 0:
+        last = ctxs[view_of(args.steps - 1)]
+        dump["resident_nodes"] = last.get_nodes()
+        dump["resident_depth"] = last.get_depth()
+        dump["resident_stats"] = np.array([st[k] for k in DUMP_STATS], np.float64)
 
     # ---- end-to-end arm ---------------------------------------------------
     barrier()
@@ -473,6 +481,8 @@ def run_product(args):
         pix_e2e += st["pixel_iterations"]
     barrier()
     wall_e2e = time.perf_counter() - t0
+    if args.dump_outputs and args.steps > 0:
+        dump["e2e_nodes"] = nodes_out.copy()
 
     # ---- end-to-end, two host threads per GPU ---------------------------------
     # The reference's host runs one view per pool thread (app/smvsrecon.cc:
@@ -530,7 +540,8 @@ def run_product(args):
     configs = {}
     if extras:
         configs = run_extra_configs(args, api, torch, dist, rank, world, local, pool_s,
-                                    ctxs, pin, barrier, reduce, hbm_peak, peak_source, small_s)
+                                    ctxs, pin, barrier, reduce, hbm_peak, peak_source, small_s,
+                                    dump)
 
     if rank == 0:
         value = pix_all / (t_dev_ms_max * 1e-3) / 1e6
@@ -604,6 +615,8 @@ def run_product(args):
             "wall_s_resident": wall_resident,
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, dump)
     for c in ctxs:
         c.close()
     if world > 1:
@@ -612,10 +625,10 @@ def run_product(args):
 
 
 def run_extra_configs(args, api, torch, dist, rank, world, local, pool_s, ctxs, pin,
-                      barrier, reduce, hbm_peak, peak_source, small_s):
+                      barrier, reduce, hbm_peak, peak_source, small_s, dump):
     """BASELINE.json configs[2], [3], [4] -> the `configs` sub-dict."""
     out = {}
-    steps = max(2, min(args.steps, 8))
+    steps = max(args.steps, 1)
     for wl in pool_s:
         wl.scene.images = [pin(a) for a in wl.scene.images]
     # the shading views re-use the contexts of the headline pool
@@ -644,6 +657,8 @@ def run_extra_configs(args, api, torch, dist, rank, world, local, pool_s, ctxs, 
         acc["rows"] += st["cg_row_iterations"]
         acc["split"] += [st["ms_construct"], st["ms_solve"], st["ms_update"]]
     barrier()
+    if args.dump_outputs:
+        dump["shading_nodes"] = ctxs[(rank + steps - 1) % len(pool_s)].get_nodes()
     (ms_max,), (pix_all,) = reduce([acc["ms"]], [acc["pix"]])
     if rank == 0:
         out["shading"] = {
@@ -716,7 +731,7 @@ def run_extra_configs(args, api, torch, dist, rank, world, local, pool_s, ctxs, 
     # ---- configs[3]: SGM (rank 0, N = 1 only: it does not shard) -----------
     if world == 1:
         try:
-            out["sgm"] = sgm_config(args, api, hbm_peak, peak_source)
+            out["sgm"] = sgm_config(args, api, hbm_peak, peak_source, dump)
         except Exception as exc:      # noqa: BLE001
             out["sgm"] = {"error": str(exc)}
 
@@ -735,7 +750,7 @@ def run_extra_configs(args, api, torch, dist, rank, world, local, pool_s, ctxs, 
     return out
 
 
-def sgm_config(args, api, hbm_peak, peak_source):
+def sgm_config(args, api, hbm_peak, peak_source, dump):
     """configs[3]: SGM 1920x1080, 128 planes, P1 = 6, P2 = 96, 8 paths. Unit:
     Mvoxel/s (265.4 M voxels per run). Algorithmic bytes per voxel (SURVEY.md
     section 8d): 11 = cost write 1 + 8 path reads + final sum write 2."""
@@ -747,7 +762,7 @@ def sgm_config(args, api, hbm_peak, peak_source):
     nvox = WIDTH * HEIGHT * 128
     for _ in range(3):
         r = api.sgm(sc.images[0], sc.images[1], M, t, dmin, dmax, 128)
-    reps = max(3, min(args.steps, 10))
+    reps = max(args.steps, 1)
     ms = np.zeros(3)
     t0 = time.perf_counter()
     for _ in range(reps):
@@ -755,6 +770,8 @@ def sgm_config(args, api, hbm_peak, peak_source):
         ms += r["ms"]
     wall = time.perf_counter() - t0
     ms /= reps
+    if args.dump_outputs:
+        dump["sgm_depth"] = r["depth"]
     dev_ms = float(ms.sum())
     out = {"workload": "configs[3]: sgm_stereo init, 1920x1080, 128 planes, 8-path aggregation "
                        "(cost volume + aggregation + WTA of one main/neighbour pair)",
@@ -789,6 +806,17 @@ def sgm_config(args, api, hbm_peak, peak_source):
     return out
 
 
+def write_outputs(path, arrays):
+    """DIR/<name>.npy of each output, float32 / float64 as computed."""
+    os.makedirs(path, exist_ok=True)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: outputs of {total} bytes exceed {DUMP_LIMIT}")
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -798,6 +826,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true",
                     help="skip the `configs` sub-dict (BASELINE.json configs[2..4])")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last step of each timed "
+                         "path returned to DIR/<name>.npy: resident_nodes / resident_depth / "
+                         "resident_stats (headline loop), e2e_nodes, and with the configs "
+                         "shading_nodes and sgm_depth; the inputs are seeded, so two builds "
+                         "can be compared output for output")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

@@ -14,10 +14,10 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "_ref", "libsmvs_ref.so")
 
 # The same C driver (oracle/ref_driver.cc) is also linked into
-# integration/_build/libsmvs_ref_b200.so, where the reference's host code runs
-# with the GPU hot path patched in (integration/Makefile).
-INTEGRATION_LIB_PATH = os.path.join(os.path.dirname(_HERE), "integration", "_build",
-                                    "libsmvs_ref_b200.so")
+# _ref/integration/libsmvs_ref_b200.so, where the reference's host code runs
+# with the GPU hot path patched in (integration/Makefile). It sits under _ref/
+# so that it goes wherever the reference build goes.
+INTEGRATION_LIB_PATH = os.path.join(_HERE, "_ref", "integration", "libsmvs_ref_b200.so")
 _libs = {}
 
 

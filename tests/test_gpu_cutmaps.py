@@ -117,7 +117,7 @@ def test_cut_depth_maps_equal_to_reference(n, w, h):
 
 @pytest.mark.gpu
 @pytest.mark.skipif(not os.path.exists(oref.INTEGRATION_LIB_PATH),
-                    reason="integration/_build not built")
+                    reason="oracle/_ref/integration not built")
 def test_cut_depth_maps_drop_in_member():
     """MeshGenerator::cut_depth_maps of the drop-in build (integration/
     b200_mesh_generator.cc: the reference's MeshGenerator object, cameras and

@@ -4,7 +4,7 @@ compiled-verbatim reference (oracle/_ref):
   * the whole inner Newton loop (lib/depth_optimizer.cc:204-304) at
     1920x1080, 6 neighbours, scale 2, without and with -S;
   * DepthOptimizer::optimize() at 1920x1080 -o2 / -o2 -S through the drop-in
-    build (integration/_build) against the pure-CPU build;
+    build (oracle/_ref/integration) against the pure-CPU build;
   * SGM 1920x1080x128: cost volume, aggregated volume and depth bit-exact.
 
 The CPU sides take 45 s .. 2.5 min on one host core each. They are started
@@ -133,7 +133,7 @@ def test_full_size_newton_loop(cpu_results, shading):
 
 
 @pytest.mark.skipif(not os.path.exists(oref.INTEGRATION_LIB_PATH),
-                    reason="integration/_build not built")
+                    reason="oracle/_ref/integration not built")
 @pytest.mark.parametrize("shading", [False, True])
 def test_full_size_optimize(cpu_results, shading):
     """The reference's own DepthOptimizer::optimize() (ladder 5 -> 2, all host

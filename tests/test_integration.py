@@ -14,7 +14,7 @@ from oracle import ref as oref
 pytestmark = [pytest.mark.gpu,
               pytest.mark.skipif(not (oref.available()
                                       and os.path.exists(oref.INTEGRATION_LIB_PATH)),
-                                 reason="oracle/_ref or integration/_build not built")]
+                                 reason="oracle/_ref or oracle/_ref/integration not built")]
 
 
 def _run(scene, lib_path, shading):

@@ -4,10 +4,80 @@
 The oracle is used here only as the checker."""
 from __future__ import annotations
 
+import atexit
+import hashlib
+import os
+
 import numpy as np
 
 from smvs_b200 import api, synth
 from oracle import ref as oref
+
+REF_OUTPUTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden",
+                           "ref_outputs.npz")
+_recorded = {}
+
+
+def _digest(a):
+    """SHA-256 of an array's shape and values (integers widened to int64,
+    floats to float64, -0 as 0): equal digests <=> np.array_equal."""
+    a = np.asarray(a)
+    if a.dtype.kind == "f":
+        a = np.where(np.isnan(a), np.nan, a.astype(np.float64) + 0.0)
+    else:
+        a = a.astype(np.int64)
+    h = hashlib.sha256(repr(a.shape).encode())
+    h.update(np.ascontiguousarray(a).tobytes())
+    return np.frombuffer(h.digest(), np.uint8)
+
+
+def _write_recorded(path):
+    old = dict(np.load(REF_OUTPUTS)) if os.path.exists(REF_OUTPUTS) else {}
+    old.update(_recorded)
+    np.savez_compressed(path, **old)
+
+
+class RefOutputs:
+    """What a test compares against the compiled reference: computed live when
+    oracle/_ref is built, else read from tests/golden/ref_outputs.npz. Large
+    outputs are stored as digests, which is all a comparison for equality
+    needs. SMVSB_RECORD_REF=<file> writes the live values of a run, merged with
+    the stored ones, to <file> (regenerate the fixture after a change of the
+    inputs of these tests)."""
+
+    def __init__(self, test):
+        self.test = test
+        self.live = oref.available()
+        self.stored = None
+        if not self.live:
+            if not os.path.exists(REF_OUTPUTS):
+                raise RuntimeError(f"neither oracle/_ref nor {REF_OUTPUTS}")
+            self.stored = np.load(REF_OUTPUTS)
+        rec = os.environ.get("SMVSB_RECORD_REF")
+        if self.live and rec and not _recorded:
+            atexit.register(_write_recorded, rec)
+
+    def _key(self, key):
+        return f"{self.test}/{key}"
+
+    def array(self, key, fn):
+        """A small reference output the test uses as an input: stored whole."""
+        if not self.live:
+            return self.stored[self._key(key)]
+        a = np.asarray(fn())
+        if os.environ.get("SMVSB_RECORD_REF"):
+            _recorded[self._key(key)] = a
+        return a
+
+    def assert_equal(self, key, out, fn):
+        """out equals the reference's output fn() element for element."""
+        if not self.live:
+            assert np.array_equal(_digest(out), self.stored[self._key(key) + "#sha256"]), key
+            return
+        ref = fn()
+        assert np.array_equal(out, ref), key
+        if os.environ.get("SMVSB_RECORD_REF"):
+            _recorded[self._key(key) + "#sha256"] = _digest(ref)
 
 
 def colour_scene(width, height, n_sub, seed_index, shading=False):
